@@ -1,6 +1,6 @@
 """bench.py — DALL-E fwd+bwd tokens/sec (BASELINE.json metric) on N x B200, and the reference arm on the host CPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c1] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c1] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = `loss = dalle(text, image_ids, return_loss=True); loss.backward()` on one synthetic batch (reference
@@ -12,12 +12,14 @@ all-reduce (dalle_pytorch_b200.distributed).  Prints ONE JSON line (rank 0).
           the loss inside every timed step
   roofline  the tcgen05 GEMM family (dominant kernel): algorithmic FLOPs of every launch / CUDA-event time of those
           launches inside the timed region, against MEASURED_PEAKS.json bf16_tflops_sustained
-  cpu_baseline  the UNMODIFIED reference (baseline/_ref, its own DALLE(...) API) on the host cores, on a bounded sample (batch 1
+  cpu_baseline  the UNMODIFIED reference (oracle/_ref, its own DALLE(...) API) on the host cores, on a bounded sample (batch 1
           of the same configuration, best of a few thread counts); the oracle port only if the reference cannot be imported
   gpu_eager_baseline  the same unmodified reference module on cuda:0 with torch's eager kernels under bf16 autocast, same batch --
           the practical GPU baseline
   extra_configs  BASELINE.json configs[2], [3] (one GPU) / configs[4] (eight GPUs) timed in the same run
 `--impl reference` times the unmodified reference on the host CPU for K steps of a batch-1 sample of the configuration.
+`--dump-outputs DIR` writes what the headline step returned in its last timed step (see output_snapshot) so that two builds can be
+compared output for output: weights and token ids come from fixed seeds, so the inputs are the same on every run.
 """
 import argparse
 import json
@@ -43,6 +45,7 @@ NUM_TEXT_TOKENS, NUM_IMAGE_TOKENS = 10000, 8192
 # of a C2 step (algorithmic operand+result bytes of the same launches: 226 MB per launch)
 GEMM_DRAM_BYTES_PER_LAUNCH = 229e6
 METRIC = 'DALL-E fwd+bwd tokens/sec at seq=1280, dim=1024'
+DUMP_BYTES = 60 * 2 ** 20      # gradient samples of --dump-outputs; with the .npy headers and the loss the files stay below 64 MB
 
 
 def log(msg):
@@ -169,7 +172,7 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------------------------
-# Reference legs: the UNMODIFIED reference (baseline/_ref or /root/reference, imported through oracle/ref_import.py with
+# Reference legs: the UNMODIFIED reference (oracle/_ref, built by oracle/build_ref.py; imported through oracle/ref_import.py with
 # the dependency shims under oracle/shims) driven through its own public API -- DALLE(...)(text, image, return_loss=True);
 # loss.backward() (train_dalle.py:609-616).  If the reference cannot be imported the oracle port is timed instead and the
 # line says kind = "port".
@@ -304,7 +307,7 @@ def run_reference_arm(args):
         step()
     dt = time.perf_counter() - t0
     val = tokens * args.steps / dt
-    what = ('unmodified reference DALLE (baseline/_ref) through its public API' if kind == 'reference'
+    what = ('unmodified reference DALLE (oracle/_ref) through its public API' if kind == 'reference'
             else 'oracle port of the reference (oracle/dalle_oracle.py)')
     sample = (f'{what}: each step = fwd+bwd on a bounded sample, batch 1 of the configuration\'s {c["batch"]} ({tokens} tokens), full '
               f'depth, fp32, torch CPU with {cores} threads (best of {sorted(seen)})')
@@ -338,6 +341,34 @@ def model_flops_per_token(c):
     n_text_pos, n_img_pos = c['text_seq_len'], c['fmap'] ** 2
     head = 2.0 * d * (n_text_pos * (NUM_TEXT_TOKENS + c['text_seq_len']) + n_img_pos * NUM_IMAGE_TOKENS) / seq
     return 3 * (c['depth'] * (32.0 * d * d + attn_flops) + head)
+
+
+def named_grads(model):
+    return [(k, p.grad) for k, p in model.named_parameters() if p.grad is not None]
+
+
+def output_snapshot(loss, grads):
+    """What a caller of one fwd+bwd step receives, on the host: the loss (float64) and every parameter gradient (float32).  A
+    gradient larger than its share of DUMP_BYTES is a sample at fixed flat indices (seeded by the parameter name, sorted)."""
+    import zlib
+    import torch
+    cap = DUMP_BYTES // 4 // max(1, len(grads))
+    out = {'loss': loss.detach().double().cpu().numpy()}
+    for k, g in grads:
+        f = g.detach().reshape(-1)
+        if f.numel() > cap:
+            idx = torch.randperm(f.numel(), generator=torch.Generator().manual_seed(zlib.crc32(k.encode())))[:cap].sort().values
+            f = f[idx.to(f.device)]
+        out['grad.' + k] = f.float().cpu().numpy()
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+    log(f'dumped {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 2 ** 20:.1f} MB) to {out_dir}')
 
 
 def measure_config(cfg_name, args, ctx, steps, want_e2e=True, want_clocks=True, batch=None, dtype_name=None):
@@ -374,6 +405,9 @@ def measure_config(cfg_name, args, ctx, steps, want_e2e=True, want_clocks=True, 
     image_h = torch.randint(0, NUM_IMAGE_TOKENS, (batch, c['fmap'] ** 2), generator=g).pin_memory()
     text_d, image_d = text_h.to(dev), image_h.to(dev)
     head_autocast = dtype == torch.bfloat16
+    dump = args.dump_outputs is not None and cfg_name == args.config and rank == 0
+    graph_leg = world == 1 and not args.no_graph
+    last = {}
 
     def zero():
         if reducer is not None:
@@ -389,6 +423,8 @@ def measure_config(cfg_name, args, ctx, steps, want_e2e=True, want_clocks=True, 
         loss.backward()
         if reducer is not None:
             reducer.finish()
+        if dump:
+            last['loss'] = loss.detach()      # detached: a kept autograd graph would break the CUDA-graph capture that follows
         return loss
 
     def barrier():
@@ -425,10 +461,19 @@ def measure_config(cfg_name, args, ctx, steps, want_e2e=True, want_clocks=True, 
     launches = ops.launches() - n0
     gemm_stats = ops.gemm_timing(False)
     clocks = sampler.stop() if (rank == 0 and want_clocks) else None
+    outputs = None
+    if dump:
+        # only the path that becomes the headline is copied out: the eager step when no graph leg follows (now, before later steps
+        # reuse the data-parallel gradient buffers), otherwise the references are kept until the graph leg is timed.  They stay the
+        # eager step's values because GraphedStep._zero and the e2e steps' zero() set p.grad = None (fresh tensors afterwards)
+        # instead of zeroing the old ones in place; a change to in-place zeroing there must snapshot here instead.
+        eager_out = (last['loss'], named_grads(model))
+        if not graph_leg:
+            outputs = output_snapshot(*eager_out)
     log(f'{cfg_name}: device-resident {ms_dev / steps:.2f} ms/step')
     res = {'cfg': cfg_name, 'c': c, 'batch': batch, 'seq': seq, 'dtype': dtype, 'ms_dev': ms_dev, 'steps': steps, 'launches': launches,
            'gemm_stats': gemm_stats, 'clocks': clocks, 'peak_mem_gb': torch.cuda.max_memory_allocated() / 2 ** 30,
-           'h2d': int(text_h.numel() * 8 + image_h.numel() * 8)}
+           'h2d': int(text_h.numel() * 8 + image_h.numel() * 8), 'outputs': outputs}
     if dtype == torch.bfloat16 and gemm_stats['simt']['launches'] != 0:
         raise RuntimeError(f"{cfg_name}: {gemm_stats['simt']['launches']} GEMM launches fell back to the fp32 CUDA-core kernel in bf16 mode "
                            '(mis-aligned operand?) -- the measured step is not the tcgen05 path')
@@ -442,12 +487,14 @@ def measure_config(cfg_name, args, ctx, steps, want_e2e=True, want_clocks=True, 
         res['ms_e2e'] = timed(e2e_step, steps)
         log(f"{cfg_name}: e2e {res['ms_e2e'] / steps:.2f} ms/step")
     # ---- the same step captured into ONE CUDA graph and replayed (single process): no Python / ctypes between the kernels ----
-    if world == 1 and not args.no_graph:
+    if graph_leg:
         try:
             step = D.GraphedStep(model, text_d, image_d, autocast_bf16=head_autocast)
             for _ in range(2):
                 step()
             ms_g = timed(lambda: step(), steps)
+            if dump and ms_g <= ms_dev:                     # run_gpu_arm's headline rule: the replay when it is not slower
+                res['outputs'] = output_snapshot(step.loss, named_grads(model))
             g = {'ms_dev': ms_g, 'kernels_per_step': step.kernels_per_step}
             if want_e2e:
                 def e2e_graph():
@@ -463,6 +510,8 @@ def measure_config(cfg_name, args, ctx, steps, want_e2e=True, want_clocks=True, 
             log(f'{cfg_name}: CUDA-graph capture failed ({type(ex).__name__}: {str(ex)[:200]}); eager numbers stand')
             res['graph'] = {'error': f'{type(ex).__name__}: {str(ex)[:200]}'}
             torch.cuda.synchronize()
+    if dump and res['outputs'] is None:                     # the eager step is the headline
+        res['outputs'] = output_snapshot(*eager_out)
     if args.with_optimizer and cfg_name == args.config:
         # full training step of the reference trainer (train_dalle.py:609-619): fwd + bwd + clip_grad_norm_(0.5) + Adam
         opt = D.FusedAdam(model.parameters(), lr=3e-4, max_grad_norm=0.5, reducer=reducer)
@@ -633,6 +682,8 @@ def run_gpu_arm(args):
     # headline = the product's execution path: the captured step when the capture succeeded and is not slower, eager otherwise
     ms_dev = gr['ms_dev'] if graphed else ms_eager
     ms_e2e = gr.get('ms_e2e', ms_e2e_eager) if graphed else ms_e2e_eager
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, main_res['outputs'])
     tokens_per_step = batch * seq * world
     value = tokens_per_step * args.steps / (ms_dev / 1e3)
     e2e_value = tokens_per_step * args.steps / (ms_e2e / 1e3)
@@ -674,7 +725,7 @@ def run_gpu_arm(args):
         what = f'batch 1 of {batch} ({seq} tokens), full depth, fwd+bwd, fp32'
         try:
             j = sub('--cpu-sample', 420)
-            src = 'unmodified reference DALLE (baseline/_ref)' if j['kind'] == 'reference' else 'oracle/dalle_oracle.py (port)'
+            src = 'unmodified reference DALLE (oracle/_ref)' if j['kind'] == 'reference' else 'oracle/dalle_oracle.py (port)'
             cpu = {'value': j['value'], 'unit': 'tokens/s', 'cores': j['cores'], 'kind': j['kind'],
                    'sample': f"{j['steps']} step(s) on {what}, {src} on {j['cores']} torch threads ({j['seconds']:.1f} s/step; tried {j['threads_tried']})"}
         except Exception as ex:   # timeout / parse failure: report the failure, keep the GPU numbers
@@ -729,6 +780,9 @@ def main():
     ap.add_argument('--extra', default=None,
                     help='comma-separated extra configurations timed in the same run and reported under "extra_configs" '
                          "(default: c3,c4 on one GPU, c5 on eight; '' = none)")
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the loss and (sampled) parameter gradients of the last step of the headline '
+                         'path as DIR/<name>.npy (float64 loss, float32 gradients, < 64 MB in all)')
     ap.add_argument('--cpu-sample', action='store_true', help=argparse.SUPPRESS)
     ap.add_argument('--gpu-eager-sample', action='store_true', help=argparse.SUPPRESS)
     args = ap.parse_args()

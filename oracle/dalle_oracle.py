@@ -5,10 +5,11 @@ BASELINE.json `north_star` (SURVEY.md §8a / Appendix A).  It is deliberately wr
 style from the reference (explicit allowed-key predicates and index arithmetic instead of
 einops/einsum reshapes) so that agreement between the two is evidence, not tautology.
 
-Parity status: PINNED against the live reference.  `oracle/make_golden.py` imports the unmodified
-reference from /root/reference (with the dependency shims under oracle/shims) and writes golden
-tensors to tests/golden/*.pt; `tests/test_oracle_vs_golden.py` checks this file against those
-fixtures (and against the live reference when /root/reference is present).  One dependency of the
+Parity status: PINNED against the reference.  `oracle/make_golden.py` imports the unmodified
+reference (oracle/ref_import.py, with the dependency shims under oracle/shims) and writes golden
+tensors to tests/golden/*.pt: whole models, and single reference modules (ref_modules.pt: sparse
+attention classes, token shift, static masks); `tests/test_oracle_vs_golden.py` checks this file
+against those fixtures.  One dependency of the
 reference, `rotary-embedding-torch`, is un-vendored and unpinned (reference setup.py:29); its two
 functions are restated from the published algorithm in oracle/shims/rotary_embedding_torch.py and
 here (`rotary_angle_table`, `apply_rotary`), so the rotary part is "pinned to the restated library",
@@ -498,3 +499,16 @@ def make_inputs(cfg: OracleConfig, batch: int, seed: int = 1, pad_tail: bool = T
             text[bi, cfg.text_seq_len - k:] = 0
     image = torch.randint(0, cfg.num_image_tokens, (batch, cfg.image_seq_len), generator=g)
     return text, image
+
+
+def make_attention_inputs(dim: int, heads: int, dim_head: int, batch: int, n: int, seed: int = 0):
+    """Deterministic weights of one attention module (to_qkv.weight, to_out.0.weight, to_out.0.bias; the reference's
+    default-init distributions) and its input x [batch, n, dim], from a private torch.Generator."""
+    g = torch.Generator().manual_seed(seed)
+    inner = heads * dim_head
+
+    def uni(shape, fan_in):
+        return (torch.rand(shape, generator=g, dtype=torch.float64) * 2 - 1).div(fan_in ** 0.5).float()
+
+    w_qkv, w_out, b_out = uni((3 * inner, dim), dim), uni((dim, inner), inner), uni((dim,), inner)
+    return w_qkv, w_out, b_out, torch.randn(batch, n, dim, generator=g, dtype=torch.float64).float()

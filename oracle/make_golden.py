@@ -123,6 +123,46 @@ def run_variant(R, name, base, over, batch, full_store, seed=0):
     return rec
 
 
+def reference_modules(R):
+    """Outputs of single reference modules for the module-level pins of tests/test_oracle_vs_golden.py: the axial and
+    conv-like sparse attention classes, PreShiftToken, and the static axial masks of the reference Transformer.  Weights
+    and inputs come from seeded generators (dalle_oracle.make_attention_inputs, torch.Generator), so only the reference's
+    outputs and a checksum of each input are stored."""
+    from dalle_oracle import make_attention_inputs, rotary_angle_table
+    rec = {'axial': {}, 'conv_like': {}, 'token_shift': {}, 'static_masks': {}, 'torch_version': torch.__version__}
+
+    def attn_record(m, dim, heads, n, text_len, fmap, seed):
+        w_qkv, w_out, b_out, x = make_attention_inputs(dim, heads, 64, 2, n, seed=seed)
+        with torch.no_grad():
+            m.to_qkv.weight.copy_(w_qkv)
+            m.to_out[0].weight.copy_(w_out)
+            m.to_out[0].bias.copy_(b_out)
+            out = m(x, rotary_pos_emb=rotary_angle_table(text_len, fmap, 64)[None])
+        return {'out': out, 'checksum': sum(float(t.double().sum()) for t in (w_qkv, w_out, b_out, x))}
+
+    dim, heads, fmap, text_seq = 64, 2, 4, 8
+    seq_len = text_seq + fmap * fmap
+    for kind, axis in (('axial_row', 0), ('axial_col', 1)):
+        for stable in (False, True):
+            for n in (24, 19):
+                m = R.SparseAxialCausalAttention(dim, seq_len, image_size=fmap, axis=axis, heads=heads, dim_head=64, stable=stable)
+                rec['axial'][(kind, stable, n)] = attn_record(m, dim, heads, n, seq_len - fmap * fmap + 1, fmap, seed=n)
+    dim, heads, fmap, text_seq = 64, 2, 6, 5
+    seq_len = text_seq + fmap * fmap
+    for kernel_size, dilation in ((3, 1), (5, 1), (3, 2)):
+        m = R.SparseConvCausalAttention(dim, seq_len, image_size=fmap, kernel_size=kernel_size, dilation=dilation, heads=heads, dim_head=64)
+        rec['conv_like'][(kernel_size, dilation)] = attn_record(m, dim, heads, seq_len, text_seq + 1, fmap, seed=kernel_size + 10 * dilation)
+    fmap, text_seq, dim = 4, 8, 32
+    seq_len = text_seq + fmap * fmap
+    sh = R.transformer.PreShiftToken(lambda x, **kw: x, image_size=fmap, seq_len=seq_len)
+    for n in (seq_len, seq_len - 3, text_seq + 1, 5):
+        rec['token_shift'][n] = sh(torch.randn(2, n, dim, generator=torch.Generator().manual_seed(n)))
+    t = R.Transformer(dim=64, depth=1, seq_len=24, heads=2, dim_head=64, image_fmap_size=4, attn_types=('full',))
+    for kind in ('axial_row', 'axial_col'):
+        rec['static_masks'][kind] = t._get_attention_mask(kind).clone()
+    return rec
+
+
 def main():
     torch.manual_seed(0)
     torch.set_num_threads(max(1, os.cpu_count() or 1))
@@ -136,6 +176,10 @@ def main():
         path = os.path.join(OUT, name + '.pt')
         torch.save(rec, path)
         print(f'{name}: loss={float(rec["loss"]):.6f} ref_time={rec["ref_seconds"]:.3f}s -> {os.path.getsize(path)/1e6:.2f} MB')
+    if not only or 'ref_modules' in only:
+        path = os.path.join(OUT, 'ref_modules.pt')
+        torch.save(reference_modules(R), path)
+        print(f'ref_modules -> {os.path.getsize(path) / 1e6:.2f} MB')
 
 
 if __name__ == '__main__':

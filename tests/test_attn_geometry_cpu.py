@@ -2,7 +2,7 @@
 column bit masks, tile-skip and tile-full tests, gathered-axial index maps and segment tiles) checked on the host: the header is
 plain C++ apart from the CUDA keywords, so g++ compiles it against a stub `common.cuh` (tests/host/) and a driver walks a grid of
 ragged geometries exhaustively (hundreds of thousands of tiles, every bit compared with the element predicate); the element
-predicate itself is compared with the CPU oracle's `allowed_mask`, which tests/test_oracle_vs_golden.py pins to the live reference.
+predicate itself is compared with the CPU oracle's `allowed_mask`, which tests/test_oracle_vs_golden.py pins to the reference's stored outputs.
 The GPU tests can only sample geometries; a wrong bit here would be silently wrong attention for some (text_len, fmap, kernel)."""
 import os
 import shutil

@@ -94,9 +94,8 @@ def cpu_kernels(monkeypatch):
     monkeypatch.setattr(ops, 'gemm_resid', _gemm_resid)
     monkeypatch.setattr(ops, 'gemm_geglu', _gemm_geglu)
     monkeypatch.setattr(decode, 'WARMUP_STEPS', 10 ** 9)            # never capture: every step runs the device-indexed code eagerly
-    D.set_compute_dtype(torch.float32)
-    yield
-    D.set_compute_dtype(torch.bfloat16)
+    with D.compute_dtype_ctx(torch.float32):                         # restores the caller's mode: later tests rely on the fp32 default
+        yield
 
 
 def _model(attn_types=('full',), shift_tokens=True, stable=False, optimize=False, depth=2, sandwich=False):

@@ -1,5 +1,5 @@
-"""Drop-in test: the UNMODIFIED reference `dalle_pytorch.DALLE` (baseline/_ref on the GPU box, /root/reference in the dev
-container) built after `patch_dalle_pytorch()` runs its block stack on libdalle_b200 and reproduces the golden vectors that the
+"""Drop-in test: the UNMODIFIED reference `dalle_pytorch.DALLE` (oracle/_ref, copied there by `build()` through
+oracle/build_ref.py) built after `patch_dalle_pytorch()` runs its block stack on libdalle_b200 and reproduces the golden vectors that the
 same reference produced on the CPU with its own blocks (rtol 1e-3 / atol 1e-5, fp32 parity mode)."""
 import pytest
 import torch
@@ -17,7 +17,7 @@ RTOL, ATOL = 1e-3, 1e-5
 def test_patched_reference_reproduces_goldens(name):
     import ref_import
     if not ref_import.reference_available():
-        pytest.skip('reference install (baseline/_ref) not present')
+        pytest.skip('reference not built into oracle/_ref')
     import dalle_pytorch_b200 as D
     from dalle_pytorch_b200 import ops
     ref = ref_import.import_reference()
