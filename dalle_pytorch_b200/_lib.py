@@ -118,6 +118,8 @@ def _declare(lib):
     lib.dalle_b200_split_bf16x3.argtypes = [c_void_p, c_void_p, c_int64, c_int, c_int, c_int, c_void_p]
     lib.dalle_b200_resid_scale.argtypes = [c_void_p, c_int, c_void_p, c_void_p, c_float, c_void_p, c_int64, c_int, c_void_p]
     lib.dalle_b200_sample_topk_gumbel.argtypes = [c_void_p, c_int, c_int, c_int, c_int64, c_int, c_float, c_void_p, ctypes.c_uint64, ctypes.c_uint64, c_void_p, c_void_p]
+    lib.dalle_b200_sample_guided_topk_gumbel.argtypes = [c_void_p, c_void_p, c_int, c_int, c_int, c_int64, c_float, c_int, c_float, c_void_p, ctypes.c_uint64, ctypes.c_uint64,
+                                                          c_void_p, c_void_p]
     lib.dalle_b200_decode_shift.argtypes = [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]
     lib.dalle_b200_decode_kv_append.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]
     lib.dalle_b200_dropout.argtypes = [c_void_p, c_void_p, c_int, c_int64, c_float, ctypes.c_uint64, ctypes.c_uint64, c_void_p]
@@ -158,5 +160,5 @@ def check(rc, what=''):
 
 EXPORTED = ['dalle_b200_version', 'dalle_b200_last_error', 'dalle_b200_device_ok', 'dalle_b200_abi_sizes',
             'dalle_b200_ln_shift_fwd', 'dalle_b200_ln_shift_bwd', 'dalle_b200_gemm', 'dalle_b200_gemm_select', 'dalle_b200_attn_fwd',
-            'dalle_b200_attn_bwd', 'dalle_b200_scale_bwd', 'dalle_b200_colsum', 'dalle_b200_qkv_rotary', 'dalle_b200_geglu_bwd', 'dalle_b200_ce_fwd', 'dalle_b200_ce_bwd', 'dalle_b200_cast_bf16', 'dalle_b200_mc_add', 'dalle_b200_split_bf16x3', 'dalle_b200_resid_scale', 'dalle_b200_dropout', 'dalle_b200_sample_topk_gumbel', 'dalle_b200_decode_shift', 'dalle_b200_decode_kv_append', 'dalle_b200_geglu_fwd',
+            'dalle_b200_attn_bwd', 'dalle_b200_scale_bwd', 'dalle_b200_colsum', 'dalle_b200_qkv_rotary', 'dalle_b200_geglu_bwd', 'dalle_b200_ce_fwd', 'dalle_b200_ce_bwd', 'dalle_b200_cast_bf16', 'dalle_b200_mc_add', 'dalle_b200_split_bf16x3', 'dalle_b200_resid_scale', 'dalle_b200_dropout', 'dalle_b200_sample_topk_gumbel', 'dalle_b200_sample_guided_topk_gumbel', 'dalle_b200_decode_shift', 'dalle_b200_decode_kv_append', 'dalle_b200_geglu_fwd',
             'dalle_b200_axpby', 'dalle_b200_embed_fwd', 'dalle_b200_embed_bwd', 'dalle_b200_sumsq', 'dalle_b200_adam', 'dalle_b200_debug_attn_timeline']

@@ -55,6 +55,9 @@ int resid_scale_launch(const void* y, int dtype, const float* resid, const float
 int mc_add_launch(const float* src, void* mc_dst, int64_t count, float scale, cudaStream_t st);
 int sample_topk_gumbel_launch(const void* logits, int dtype, int rows, int vocab, long long ld, int k, float temperature, const float* gumbel,
                               unsigned long long seed, unsigned long long offset, long long* out, cudaStream_t st);
+int sample_guided_topk_gumbel_launch(const void* cond, const void* null_logits, int dtype, int rows, int vocab, long long ld, float cond_scale, int k,
+                                     float temperature, const float* gumbel, unsigned long long seed, unsigned long long offset, long long* out,
+                                     cudaStream_t st);
 int dropout_launch(const void* x, void* y, int dtype, int64_t count, float p, unsigned long long seed, unsigned long long offset, cudaStream_t st);
 int geglu_fwd_launch(const float* u, float* h, int64_t rows, int hidden, cudaStream_t st);
 int axpby_launch(const float* a, const float* b, float alpha, float* y, int64_t count, cudaStream_t st);
@@ -334,6 +337,15 @@ int dalle_b200_sample_topk_gumbel(const void* logits, int dtype, int rows, int v
   DB200_CHECK_ARG(k >= 1 && k <= vocab && temperature > 0.f, "sample_topk_gumbel: need 1 <= k <= vocab and temperature > 0");
   if ((size_t)vocab * 4 > 200 * 1024) return set_error(DB200_ERR_UNSUPPORTED, "sample_topk_gumbel: vocab=%d does not fit the shared-memory row buffer", vocab);
   return sample_topk_gumbel_launch(logits, dtype, rows, vocab, ld, k, temperature, gumbel, seed, offset, reinterpret_cast<long long*>(out), (cudaStream_t)stream);
+}
+
+int dalle_b200_sample_guided_topk_gumbel(const void* cond, const void* null_logits, int dtype, int rows, int vocab, int64_t ld, float cond_scale, int k,
+                                         float temperature, const float* gumbel, uint64_t seed, uint64_t offset, int64_t* out, void* stream) {
+  DB200_CHECK_ARG(cond && null_logits && out && rows >= 0 && vocab > 0 && ld >= vocab && dtype_ok(dtype), "sample_guided_topk_gumbel: bad args");
+  DB200_CHECK_ARG(k >= 1 && k <= vocab && temperature > 0.f, "sample_guided_topk_gumbel: need 1 <= k <= vocab and temperature > 0");
+  if ((size_t)vocab * 4 > 200 * 1024) return set_error(DB200_ERR_UNSUPPORTED, "sample_guided_topk_gumbel: vocab=%d does not fit the shared-memory row buffer", vocab);
+  return sample_guided_topk_gumbel_launch(cond, null_logits, dtype, rows, vocab, ld, cond_scale, k, temperature, gumbel, seed, offset,
+                                          reinterpret_cast<long long*>(out), (cudaStream_t)stream);
 }
 
 int dalle_b200_decode_shift(const float* h, void* y, int out_dtype, int batch, int d, float* ring_top, float* ring_left, const int64_t* pos,

@@ -1290,18 +1290,35 @@ __device__ __forceinline__ uint32_t float_key(float v) {            // ascending
   return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
 
+// logit i of the sampled row: the row itself, or (guided) null + (cond - null) * s evaluated as torch evaluates
+// `null + (cond - null) * cond_scale` on tensors of dtype T -- three separately rounded operations in fp32 (no contraction), each
+// result rounded to T -- so that the guided row equals torch's guided logits bit for bit
 template <typename T>
-__global__ void __launch_bounds__(SAMPLE_THREADS) sample_topk_gumbel_kernel(const T* __restrict__ logits, int V, long long ld, int k, float inv_temp,
-                                                                           const float* __restrict__ gumbel, unsigned long long seed,
-                                                                           unsigned long long offset, long long* __restrict__ out) {
+struct PlainRow {
+  const T* p;
+  __device__ __forceinline__ float operator()(int i) const { return to_f32(p[i]); }
+};
+template <typename T>
+struct GuidedRow {
+  const T* cond; const T* null_; float s;
+  __device__ __forceinline__ float operator()(int i) const {
+    const float c = to_f32(cond[i]), u = to_f32(null_[i]);
+    const float d = to_f32(from_f32<T>(__fsub_rn(c, u)));
+    const float m = to_f32(from_f32<T>(__fmul_rn(d, s)));
+    return to_f32(from_f32<T>(__fadd_rn(u, m)));
+  }
+};
+
+template <typename Row>
+__device__ __forceinline__ void sample_topk_gumbel_row(const Row lrow, int row, int V, int k, float inv_temp, const float* __restrict__ gumbel,
+                                                       unsigned long long seed, unsigned long long offset, long long* __restrict__ out) {
   extern __shared__ uint32_t keys[];                                  // [V]
   __shared__ uint32_t hist[256];
   __shared__ uint32_t s_prefix, s_remaining;
   __shared__ float s_val[SAMPLE_THREADS / 32];
   __shared__ int s_idx[SAMPLE_THREADS / 32];
-  const int row = blockIdx.x, tid = threadIdx.x;
-  const T* lrow = logits + (long long)row * ld;
-  for (int i = tid; i < V; i += SAMPLE_THREADS) keys[i] = float_key(to_f32(lrow[i]));
+  const int tid = threadIdx.x;
+  for (int i = tid; i < V; i += SAMPLE_THREADS) keys[i] = float_key(lrow(i));
   if (tid == 0) { s_prefix = 0u; s_remaining = static_cast<uint32_t>(k); }
   __syncthreads();
   uint32_t mask = 0u;
@@ -1343,7 +1360,7 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) sample_topk_gumbel_kernel(cons
       const float u = (static_cast<float>(w >> 8) + 0.5f) * (1.0f / 16777216.0f);        // (0, 1)
       g = -logf(-logf(u + 1e-20f) + 1e-20f);                         // dalle_pytorch.py:50-52
     }
-    const float v = to_f32(lrow[i]) * inv_temp + g;
+    const float v = lrow(i) * inv_temp + g;
     if (v > best || (v == best && i < best_i)) { best = v; best_i = i; }
   }
 #pragma unroll
@@ -1359,6 +1376,26 @@ __global__ void __launch_bounds__(SAMPLE_THREADS) sample_topk_gumbel_kernel(cons
       if (s_val[w] > best || (s_val[w] == best && s_idx[w] < best_i)) { best = s_val[w]; best_i = s_idx[w]; }
     out[row] = best_i;
   }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(SAMPLE_THREADS) sample_topk_gumbel_kernel(const T* __restrict__ logits, int V, long long ld, int k, float inv_temp,
+                                                                           const float* __restrict__ gumbel, unsigned long long seed,
+                                                                           unsigned long long offset, long long* __restrict__ out) {
+  const int row = blockIdx.x;
+  sample_topk_gumbel_row(PlainRow<T>{logits + (long long)row * ld}, row, V, k, inv_temp, gumbel, seed, offset, out);
+}
+
+// classifier-free guidance: row r of the guided logits is formed from cond row r and null row r on the fly (never written); the
+// Philox counters are those of a [rows, V] guided logits tensor passed to sample_topk_gumbel_kernel
+template <typename T>
+__global__ void __launch_bounds__(SAMPLE_THREADS) sample_guided_topk_gumbel_kernel(const T* __restrict__ cond, const T* __restrict__ null_, long long ld,
+                                                                                  float cond_scale, int V, int k, float inv_temp,
+                                                                                  const float* __restrict__ gumbel, unsigned long long seed,
+                                                                                  unsigned long long offset, long long* __restrict__ out) {
+  const int row = blockIdx.x;
+  sample_topk_gumbel_row(GuidedRow<T>{cond + (long long)row * ld, null_ + (long long)row * ld, cond_scale}, row, V, k, inv_temp, gumbel, seed,
+                         offset, out);
 }
 
 int sample_topk_gumbel_launch(const void* logits, int dtype, int rows, int vocab, long long ld, int k, float temperature, const float* gumbel,
@@ -1378,6 +1415,29 @@ int sample_topk_gumbel_launch(const void* logits, int dtype, int rows, int vocab
     sample_topk_gumbel_kernel<__nv_bfloat16><<<rows, SAMPLE_THREADS, smem, st>>>(reinterpret_cast<const __nv_bfloat16*>(logits), vocab, ld, k, inv_temp, gumbel,
                                                                                seed, offset, out);
   DB200_LAUNCH_OK("sample_topk_gumbel_kernel");
+  return DB200_OK;
+}
+
+int sample_guided_topk_gumbel_launch(const void* cond, const void* null_logits, int dtype, int rows, int vocab, long long ld, float cond_scale, int k,
+                                     float temperature, const float* gumbel, unsigned long long seed, unsigned long long offset, long long* out,
+                                     cudaStream_t st) {
+  if (rows == 0) return DB200_OK;
+  const size_t smem = (size_t)vocab * 4;
+  static std::atomic<bool> attr_done{false};
+  if (!attr_done.load(std::memory_order_acquire)) {
+    DB200_CUDA_OK(cudaFuncSetAttribute(sample_guided_topk_gumbel_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    DB200_CUDA_OK(cudaFuncSetAttribute(sample_guided_topk_gumbel_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    attr_done.store(true, std::memory_order_release);
+  }
+  const float inv_temp = 1.0f / temperature;
+  if (dtype == DB200_F32)
+    sample_guided_topk_gumbel_kernel<float><<<rows, SAMPLE_THREADS, smem, st>>>(reinterpret_cast<const float*>(cond), reinterpret_cast<const float*>(null_logits),
+                                                                                ld, cond_scale, vocab, k, inv_temp, gumbel, seed, offset, out);
+  else
+    sample_guided_topk_gumbel_kernel<__nv_bfloat16><<<rows, SAMPLE_THREADS, smem, st>>>(reinterpret_cast<const __nv_bfloat16*>(cond),
+                                                                                        reinterpret_cast<const __nv_bfloat16*>(null_logits), ld, cond_scale,
+                                                                                        vocab, k, inv_temp, gumbel, seed, offset, out);
+  DB200_LAUNCH_OK("sample_guided_topk_gumbel_kernel");
   return DB200_OK;
 }
 

@@ -177,18 +177,26 @@ class DALLE(nn.Module):
         cache = {} if use_cache else None
         # graph-replayed steps (decode.py): after the prompt pass every image token is one CUDA-graph replay + the sampling launch
         graph_ok = use_cache and decode.GRAPH_DEFAULT and decode.eligible(self, text, cond_scale)
+        # classifier-free guidance on that path: the conditional and the unconditional stream as one batch of 2b sequences
+        guided = graph_ok and cond_scale != 1
+        if guided and not decode.GUIDED_DEFAULT:
+            graph_ok = guided = False
         stepper, sample = None, None
         for cur_len in range(out.shape[1], total_len):
             is_image = cur_len >= text_seq_len
             if graph_ok and stepper is None and cur_len > text_seq_len and cache.get('offset') == cur_len:
-                stepper = decode.GraphedDecoder(self, cache)
+                stepper = decode.GuidedDecoder(self, cache) if guided else decode.GraphedDecoder(self, cache)
             if stepper is not None:
                 logits = stepper.step(sample)
+            elif guided:
+                logits = decode.guided_prompt(self, out[:, :text_seq_len], out[:, text_seq_len:], cache)
             else:
                 text, image = out[:, :text_seq_len], out[:, text_seq_len:]
                 logits = self.forward_with_cond_scale(text, image, cond_scale=cond_scale, cache=cache)
                 logits = logits[:, -1, :]
-            if logits.is_cuda and logits.shape[-1] * 4 <= 200 * 1024:
+            if guided:
+                sample = decode.sample_guided(logits, cond_scale, filter_thres, temperature)
+            elif logits.is_cuda and logits.shape[-1] * 4 <= 200 * 1024:
                 # top_k + gumbel_sample (dalle_pytorch.py:533-539) as one library launch; the Philox pair follows torch's generator
                 seed, off = DropoutRNG.draw(logits.numel())
                 sample = ops.sample_topk_gumbel(logits.contiguous(), filter_thres, temperature, seed, off)

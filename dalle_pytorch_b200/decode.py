@@ -26,8 +26,18 @@ flat step (FLAT_DEFAULT) 7 953 -> + 256-key buckets (BUCKET_DEFAULT) 8 896 -> + 
 csrc/decode.cu 10 444 -> + the small-M weight-streaming GEMM (csrc/gemm_smallm.cu) 13 781 (1.16 ms per step).  One step of the first graph was 364 kernels / 2.84 ms (profiles/r02_decode_step_launches.txt:
 29 % attention over the whole buffer on 128-query tiles, 28 % the four M = 16 GEMMs per layer, 32 % torch index glue).
 
-`DALLE_B200_DECODE_GRAPH=0` restores the host-indexed loop (see GRAPH_DEFAULT); models the path does not cover (reversible executor,
-sparse-pattern layers that re-run the prefix, classifier-free guidance with cond_scale != 1) use the eager loop.
+Classifier-free guidance (cond_scale = s != 1, GuidedDecoder): the conditional and the unconditional stream are decoded as ONE batch of
+2b sequences -- rows [:b] on the real text, rows [b:] on zeroed text (what DALLE.forward(null_cond_prob=1.) makes of it), each row with
+its own cache -- so every weight byte is read once per token for both streams.  The prompt pass is one eager DALLE.forward over the
+prefix repeated twice; every later token is one replay of the same step at batch 2b, fed the sampled token in both halves, its GEMMs on
+the small-M kernel up to 32 rows (ops.small_m_rows).  dalle_b200_sample_guided_topk_gumbel forms null + (cond - null) * s from the
+[2b, V] logits and samples in one launch.  The result is classifier-free guidance as the uncached forward_with_cond_scale defines it
+(two independent forwards over the prefix): the eager cached loop instead hands the null pass a shallow copy of the conditional cache.
+tools/guided_probe.py times it against the unguided graph and the eager guided loop.
+
+`DALLE_B200_DECODE_GRAPH=0` restores the host-indexed loop (see GRAPH_DEFAULT), `DALLE_B200_DECODE_GUIDED=0` the eager loop for
+cond_scale != 1 only; models the path does not cover (reversible executor, sparse-pattern layers that re-run the prefix) use the eager
+loop.
 """
 import os
 from collections import deque
@@ -43,6 +53,8 @@ FLAT_DEFAULT = os.environ.get('DALLE_B200_DECODE_FLAT', '1') != '0'
 # the whole buffer, one graph)
 BUCKET_DEFAULT = int(os.environ.get('DALLE_B200_DECODE_BUCKET', '256'))
 WARMUP_STEPS = 2
+# classifier-free guidance (cond_scale != 1) on the graph-replayed path: GuidedDecoder, both streams as one batch of 2b sequences
+GUIDED_DEFAULT = os.environ.get('DALLE_B200_DECODE_GUIDED', '1') != '0'
 
 
 class ShiftRing:
@@ -142,7 +154,8 @@ def _flat_plan(model):
 
 
 def eligible(model, text, cond_scale):
-    return bool(text.is_cuda and cond_scale == 1 and _attention_layers(model) is not None)
+    """May generate_images(use_cache=True, cond_scale=cond_scale) decode through GraphedDecoder (cond_scale == 1) or GuidedDecoder?"""
+    return bool(text.is_cuda and _attention_layers(model) is not None)
 
 
 class GraphedDecoder:
@@ -271,3 +284,36 @@ class GraphedDecoder:
             self.graph.replay()
         self.cache['offset'] += 1
         return self.logits
+
+
+def guided_prompt(model, text, image, cache):
+    """Prompt pass of guided decoding: one DALLE.forward of the prefix for 2b sequences (rows [:b] with the text, rows [b:] with zeroed
+    text, the image prefix in both) that fills `cache` for all of them -> [2b, V] logits of the last position."""
+    return model(torch.cat((text, torch.zeros_like(text))), torch.cat((image, image)), cache=cache)[:, -1]
+
+
+class GuidedDecoder(GraphedDecoder):
+    """GraphedDecoder over the 2b-sequence cache of guided_prompt: step(sample) feeds the [b] sampled tokens to both halves and returns
+    the [2b, V] logits (conditional rows first).  The step's GEMMs of up to 32 rows run on the small-M kernel."""
+
+    def step(self, sample):
+        from . import ops
+        with ops.small_m_rows(32):
+            return super().step(sample.repeat(2))
+
+
+def sample_guided(logits, cond_scale, filter_thres, temperature):
+    """[2b, V] logits (conditional rows, then unconditional) -> [b] tokens of null + (cond - null) * cond_scale, consuming the random
+    numbers of the eager loop: the draw of DALLE.forward(null_cond_prob=1.) (prob_mask_like), then the sampling draw -- so a seed gives
+    the tokens of generate_images(use_cache=False, cond_scale=cond_scale)."""
+    from . import ops
+    from .dalle import prob_mask_like, top_k, gumbel_sample
+    from .functional import DropoutRNG
+    b, V = logits.shape[0] // 2, logits.shape[1]
+    prob_mask_like((b,), 1., device=logits.device)
+    if logits.is_cuda and V * 4 <= 200 * 1024:
+        seed, off = DropoutRNG.draw(b * V)
+        return ops.sample_guided_topk_gumbel(logits.contiguous(), cond_scale, filter_thres, temperature, seed, off)
+    null = logits[b:]
+    guided = null + (logits[:b] - null) * cond_scale
+    return gumbel_sample(top_k(guided, thres=filter_thres), temperature=temperature, dim=-1)

@@ -1,6 +1,7 @@
 """Thin torch-tensor wrappers over the C ABI (include/dalle_b200.h).  No arithmetic happens in Python:
 each function fills a POD struct with device pointers and enqueues the kernel on the current CUDA stream.
 Tensors are allocated by torch (the library never owns memory, SURVEY.md §8b)."""
+import contextlib
 import ctypes
 import os
 
@@ -139,11 +140,26 @@ def _gemm(P):
 
 
 SMALL_M = os.environ.get('DALLE_B200_SMALLM', '1') != '0'      # M <= 16 bf16 GEMMs (decoding) on the weight-streaming kernel
+_small_m_rows = 16        # row limit of the rule below; small_m_rows() raises it for the duration of a block
+
+
+@contextlib.contextmanager
+def small_m_rows(rows):
+    """Send bf16 GEMMs of up to `rows` (<= 32) rows to the weight-streaming kernel inside the block.  The guided decoder runs its
+    step at batch 2b (conditional + unconditional stream) under small_m_rows(32); everywhere else the limit stays at 16."""
+    global _small_m_rows
+    assert 1 <= rows <= 32
+    prev, _small_m_rows = _small_m_rows, rows
+    try:
+        yield
+    finally:
+        _small_m_rows = prev
 
 
 def _small_m(A, N, a_mn=False, b_mn=False):
-    """A [M, K] bf16 with M <= 16: the problem db200_gemm_backend::DB200_GEMM_SMALLM covers (csrc/gemm_smallm.cu)."""
-    return (SMALL_M and A.dtype == torch.bfloat16 and not a_mn and not b_mn and 1 <= A.shape[0] <= 16 and A.shape[1] % 256 == 0
+    """A [M, K] bf16 with M <= 16 (small_m_rows: up to 32): the problem db200_gemm_backend::DB200_GEMM_SMALLM covers
+    (csrc/gemm_smallm.cu)."""
+    return (SMALL_M and A.dtype == torch.bfloat16 and not a_mn and not b_mn and 1 <= A.shape[0] <= _small_m_rows and A.shape[1] % 256 == 0
             and N % 16 == 0)
 
 
@@ -208,6 +224,25 @@ def sample_topk_gumbel(logits, thres=0.5, temperature=1.0, seed=0, offset=0, gum
     out = torch.empty(B, device=logits.device, dtype=torch.int64)
     _lib.check(_lib.lib().dalle_b200_sample_topk_gumbel(_p(logits), dt_code(logits.dtype), B, V, logits.stride(0), k, float(temperature), _p(gumbel),
                                                         int(seed) & (2 ** 64 - 1), int(offset), _p(out), _stream()), 'sample_topk_gumbel')
+    _count()
+    return out
+
+
+def sample_guided_topk_gumbel(logits, cond_scale, thres=0.5, temperature=1.0, seed=0, offset=0, gumbel=None):
+    """logits [2b, V] = conditional rows [:b] then unconditional rows [b:] -> int64 [b]: sample_topk_gumbel of the guided logits
+    null + (cond - null) * cond_scale (forward_with_cond_scale, dalle_pytorch.py:564-574), which the kernel forms row by row
+    without writing them.  Same (seed, offset) (or `gumbel` [b, V]) -> the same tokens as torch's guided logits through
+    sample_topk_gumbel."""
+    B2, V = logits.shape
+    assert B2 % 2 == 0 and logits.stride(1) == 1
+    b = B2 // 2
+    k = max(int((1 - thres) * V), 1)
+    out = torch.empty(b, device=logits.device, dtype=torch.int64)
+    if gumbel is not None:
+        assert gumbel.shape == (b, V) and gumbel.dtype == torch.float32 and gumbel.is_contiguous()
+    _lib.check(_lib.lib().dalle_b200_sample_guided_topk_gumbel(_p(logits[:b]), _p(logits[b:]), dt_code(logits.dtype), b, V, logits.stride(0),
+                                                               float(cond_scale), k, float(temperature), _p(gumbel), int(seed) & (2 ** 64 - 1),
+                                                               int(offset), _p(out), _stream()), 'sample_guided_topk_gumbel')
     _count()
     return out
 

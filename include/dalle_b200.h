@@ -57,7 +57,8 @@ typedef enum {
   DB200_EPI_GEGLU_BWD = 4  /* du = [dh*gelu(g) | dh*a*gelu'(g)]                     autograd of the above      */
 } db200_epilogue;
 
-/* SMALLM: weight-streaming mma.sync kernel for 1 <= M <= 16 rows (decoding), bf16 K-major operands, K % 256 == 0, STORE / RESID / GEGLU;
+/* SMALLM: weight-streaming mma.sync kernel for 1 <= M <= 32 rows (decoding; M > 16 = a second 16-row A fragment, e.g. the 2b rows of
+ * classifier-free guidance), bf16 K-major operands, K % 256 == 0, STORE / RESID / GEGLU;
  * chosen explicitly by the caller (AUTO never selects it), DB200_ERR_UNSUPPORTED when the problem does not qualify */
 typedef enum { DB200_GEMM_AUTO = 0, DB200_GEMM_SIMT = 1, DB200_GEMM_TCGEN05 = 2, DB200_GEMM_SMALLM = 3 } db200_gemm_backend;
 
@@ -266,6 +267,12 @@ int dalle_b200_resid_scale(const void* y, int dtype, const float* resid, const f
  * that pointer is not NULL (tests).  logits: [rows, ld] (dtype), out: int64 [rows]. */
 int dalle_b200_sample_topk_gumbel(const void* logits, int dtype, int rows, int vocab, int64_t ld, int k, float temperature, const float* gumbel,
                                   uint64_t seed, uint64_t offset, int64_t* out, void* stream);
+/* Classifier-free guidance (generate_images(cond_scale = s)): the same sampling for the guided logits null + (cond - null) * s of
+ * rows [rows, vocab], formed element by element from cond [rows, ld] and null_logits [rows, ld] (dtype) and never written.  Each of
+ * the three operations is rounded separately (fp32, then to dtype) as torch rounds `null + (cond - null) * s`, so the result -- and
+ * with the same (seed, offset) the token -- equals dalle_b200_sample_topk_gumbel on torch's guided logits. */
+int dalle_b200_sample_guided_topk_gumbel(const void* cond, const void* null_logits, int dtype, int rows, int vocab, int64_t ld, float cond_scale, int k,
+                                         float temperature, const float* gumbel, uint64_t seed, uint64_t offset, int64_t* out, void* stream);
 /* Graph-replayed decoding (dalle_pytorch_b200/decode.py): one new token per sequence, its POSITION read from device memory (`pos`,
  * one int64) so that one captured launch sequence serves every token.
  * decode_shift: PreShiftToken's cache branch (reference transformer.py:155-170) for the token at position *pos.  h [batch, d] fp32 =
